@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W      # N ranks, NCCL
     python bench.py --impl reference --gpus 1 --steps 3 --warmup 1  # reference arm (CPU)
+    python bench.py --gpus 1 --steps 10 --warmup 3 --dump-outputs DIR   # also write the last timed step's outputs
 
 Metric (BASELINE.json): valid mel-frames/s of batched synthesis.  A "step" is one eval-mode
 `FeedForwardTransformer._forward` over one synthetic LJSpeech-shaped batch: phoneme encoder,
@@ -191,22 +192,43 @@ def cpu_frames_per_s(B: int, T: int, L: int, steps: int, warmup: int, threads: i
         kind = "reference"
 
         def fwd():
-            model._forward(bt["xs"], bt["ilens"], bt["olens"], bt["ds"].clone(), bt["es"], bt["ps"], is_inference=False)
+            return model._forward(bt["xs"], bt["ilens"], bt["olens"], bt["ds"].clone(), bt["es"], bt["ps"], is_inference=False)
     else:
         from oracle import fs2_oracle as O
         kind = "port"
 
         def fwd():
-            O.forward_path(sd, bt["xs"], bt["ilens"], bt["olens"], bt["ds"].clone(), bt["es"], bt["ps"], False)
+            return O.forward_path(sd, bt["xs"], bt["ilens"], bt["olens"], bt["ds"].clone(), bt["es"], bt["ps"], False)
     times = []
     with torch.no_grad():
         for i in range(warmup + steps):
             t0 = time.perf_counter()
-            fwd()
+            out = fwd()
             if i >= warmup:
                 times.append(time.perf_counter() - t0)
     dt = sum(times) / len(times)
-    return B * L / dt, dt, cores, kind
+    return B * L / dt, dt, cores, kind, out
+
+
+DUMP_BUDGET = 60 * 10 ** 6   # bytes of array data written by --dump-outputs: under 64 MB with the .npy headers
+
+
+def dump_outputs(directory: str, arrays) -> None:
+    """Write {name: tensor} as DIR/<name>.npy (floating point as float32, integers as float64, both exact).  When the
+    arrays exceed DUMP_BUDGET, each keeps the same share of its entries at positions drawn from a fixed seed, written
+    flattened beside DIR/<name>_index.npy; the inputs of a run are seeded, so two builds can be compared file by file."""
+    import numpy as np
+    host = {k: v.detach().to("cpu", torch.float64 if not v.is_floating_point() or v.dtype == torch.float64 else torch.float32)
+            for k, v in arrays.items()}
+    total = sum(v.numel() * v.element_size() for v in host.values())
+    os.makedirs(directory, exist_ok=True)
+    for name, v in host.items():
+        if total > DUMP_BUDGET:
+            keep = max(1, int(v.numel() * (DUMP_BUDGET / 3) / total))    # float64 indices: at most twice the values' bytes
+            idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            np.save(os.path.join(directory, f"{name}_index.npy"), idx.to(torch.float64).numpy())
+            v = v.reshape(-1)[idx]
+        np.save(os.path.join(directory, f"{name}.npy"), v.numpy())
 
 
 def run_reference(args):
@@ -217,7 +239,9 @@ def run_reference(args):
         return
     B, T, L = WORKLOADS[args.workload]
     Bs = min(B, args.cpu_sample_batch)
-    fps, dt, cores, kind = cpu_frames_per_s(Bs, T, L, args.steps, args.warmup, args.cpu_threads)
+    fps, dt, cores, kind, out = cpu_frames_per_s(Bs, T, L, args.steps, args.warmup, args.cpu_threads)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(("before_outs", "after_outs", "d_outs", "e_outs", "p_outs"), out)))
     sample = f"{Bs} of the {B} utterances of workload {args.workload} (T={T}, L={L}) per step, {cores} threads"
     line = {
         "impl": "reference", "metric": "mel-frames/sec (batched inference)", "value": fps, "unit": "frames/s",
@@ -267,8 +291,14 @@ def run_length_regulator(args):
         return e0.elapsed_time(e1) / steps
 
     n0 = lib.fs2_kernel_launches()
-    ms = timed(lambda: lr(hs_d, ds_d, il_d, alpha=4.0), args.steps, max(args.warmup, 3))
+    last_out = [None]
+
+    def step():
+        last_out[0] = lr(hs_d, ds_d, il_d, alpha=4.0)
+    ms = timed(step, args.steps, max(args.warmup, 3))
     launches = (lib.fs2_kernel_launches() - n0) // (args.steps + max(args.warmup, 3))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"out": last_out[0]})
 
     def e2e():
         o = lr(hs_h.to(dev, non_blocking=True), ds_h.to(dev, non_blocking=True), il_d, alpha=4.0)
@@ -361,6 +391,7 @@ def run_b200(args):
             args.collective = "gather"
             collective_note = f"peer_copy unavailable ({type(e).__name__}: {str(e)[:160]}); fell back to the NCCL gather"
     step_no = [0]
+    last_out = [None]           # what the last device-resident step returned (--dump-outputs)
 
     def timed(fn, steps, warmup):
         for i in range(warmup):
@@ -433,6 +464,7 @@ def run_b200(args):
                 else:
                     out = model._forward(*[devin[k] for k in keys], is_inference=False)
             collective(out[1], i)
+            last_out[0] = out
             return out[1]
 
         def step_e2e(i):
@@ -499,12 +531,20 @@ def run_b200(args):
         step(i)
     torch.cuda.synchronize()
     t_begin = time.time()
+    outputs = None
+
+    def keep_outputs():         # the last timed step's (before_outs, after_outs, d_outs, e_outs, p_outs), on the host
+        nonlocal outputs
+        if args.dump_outputs and rank == 0:
+            names = ("before_outs", "after_outs", "d_outs", "e_outs", "p_outs")
+            outputs = {n: t.to("cpu") for n, t in zip(names, last_out[0])}
+
     if args.e2e_first:                      # diagnostic: does the e2e - value gap follow the loop order (clock sag under the power cap)?
         ms_e2e = timed(step_e2e, args.steps, 2); flush()
         t_mid = time.time()
-        ms_step = timed(step, args.steps, 0); flush()
+        ms_step = timed(step, args.steps, 0); flush(); keep_outputs()
     else:
-        ms_step = timed(step, args.steps, 0); flush()
+        ms_step = timed(step, args.steps, 0); flush(); keep_outputs()
         t_mid = time.time()
         ms_e2e = timed(step_e2e, args.steps, 2); flush()
     t_end = time.time()
@@ -589,6 +629,8 @@ def run_b200(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
 
     hbm, tf_burst, tf_sus, peak_src = peaks()
     frames = frames_rank * world
@@ -658,7 +700,7 @@ def run_b200(args):
     if roof:
         line["roofline"] = roof
     if cpu:
-        cpu_fps, cpu_dt, cores, kind = cpu
+        cpu_fps, cpu_dt, cores, kind, _ = cpu
         line["cpu_baseline"] = {"value": cpu_fps, "unit": "frames/s", "cores": cores, "kind": kind,
                                 "sample": f"{min(B, args.cpu_sample_batch)} of the {B} utterances of workload {args.workload}, 1 warm-up + 1 timed forward, {cores} threads"}
     print(json.dumps(line), flush=True)
@@ -683,7 +725,12 @@ def main():
     ap.add_argument("--settle-s", type=float, default=0.5, help="idle seconds before every timed loop (same power-cap state for each)")
     ap.add_argument("--e2e-first", type=int, default=0, help="diagnostic: time the e2e loop before the device-resident loop")
     ap.add_argument("--graph", type=int, default=1, help="1: replay the step as one CUDA graph (default), 0: eager launches")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last device-resident timed step returned as DIR/<name>.npy "
+                         "(rank 0; at most 64 MB in all, a seeded sample beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

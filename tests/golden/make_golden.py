@@ -1,10 +1,10 @@
 #!/usr/bin/env python
 """Generate the golden vectors under tests/golden/ from the UNMODIFIED reference.
 
-Run in the build container only (it imports /root/reference, which does not
-exist on the GPU box):
+It needs a checkout of the reference FastSpeech2 project, given as the first
+argument; the tests themselves only read the stored fixtures:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py /path/to/FastSpeech2 [--collate-only | --filelist-only | --train-only | --dropin-only]
 
 The reference is imported through a `sys.modules` shim for five third-party
 packages its import chain touches but the model path never uses (SURVEY.md
@@ -20,7 +20,7 @@ import types
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
+REF = os.path.abspath(sys.argv[1])
 sys.path.insert(0, REPO)
 
 for name in ("librosa", "nltk", "g2p_en", "unidecode", "inflect"):
@@ -209,12 +209,97 @@ def filelist_twin():
         e_mean=(e_.double() * valid).sum(1) / olens.double(), p_mean=(p_.double() * valid).sum(1) / olens.double())
 
 
+GRAD_SAMPLES = 32      # gradient entries stored per parameter (the full gradients are ~100 MB per case)
+
+
+def train_step_fixture():
+    """`model.train(); loss, report = model(...); loss.backward()` of the reference on the CPU in fp32, with every dropout
+    mask drawn in call order from one seeded generator (tests/_synth.py).  Stored: the shape and rate of each dropout
+    call (the test redraws the same masks), the loss, the report, per parameter the max-abs and L2 norm of its gradient
+    plus GRAD_SAMPLES entries at seeded positions, and BatchNorm's updated running statistics."""
+    from fastspeech2_b200.synthetic import make_batch
+    from _synth import DROPOUT_SEED, TRAIN_CASES
+    torch.set_num_threads(min(16, os.cpu_count() or 1))
+    real = torch.nn.functional.dropout
+    for case, kw in TRAIN_CASES.items():
+        kw = dict(kw)
+        bt = make_batch(kw.pop("B"), kw.pop("T"), kw.pop("L"), **kw)
+        model, _ = build_reference()
+        model.train()
+        gen = torch.Generator().manual_seed(DROPOUT_SEED)
+        shapes, rates = [], []
+
+        def shared_dropout(input, p=0.5, training=True, inplace=False):
+            if not training or p == 0.0:
+                return input
+            m = torch.rand(input.shape, generator=gen) >= p
+            shapes.append(list(input.shape) + [1] * (4 - input.dim()))
+            rates.append((input.dim(), p))
+            return input * m.to(input.dtype) / (1.0 - p)
+
+        torch.nn.functional.dropout = shared_dropout
+        try:
+            loss, report = model(*[bt[k] for k in ("xs", "ilens", "ys", "olens", "ds", "es", "ps")])
+            loss.backward()
+        finally:
+            torch.nn.functional.dropout = real
+        pick = torch.Generator().manual_seed(0)
+        names, numel, has, maxabs, norm, off, idx, val = [], [], [], [], [], [0], [], []
+        for name, p in model.named_parameters():
+            names.append(name)
+            numel.append(p.numel())
+            has.append(p.grad is not None)
+            g = p.grad.detach().reshape(-1) if p.grad is not None else torch.zeros(0)
+            maxabs.append(float(g.abs().max()) if g.numel() else 0.0)
+            norm.append(float(g.double().norm()) if g.numel() else 0.0)
+            i = torch.randperm(g.numel(), generator=pick)[:GRAD_SAMPLES].sort().values if g.numel() else torch.zeros(0, dtype=torch.int64)
+            idx.append(i.to(torch.int32))
+            val.append(g[i])
+            off.append(off[-1] + i.numel())
+        bufs = {n: b for n, b in model.named_buffers() if "running" in n or "num_batches" in n}
+        npz(f"train_{case}", mask_shape=np.array(shapes, dtype=np.int64), mask_ndim=np.array([r[0] for r in rates]),
+            mask_p=np.array([r[1] for r in rates], dtype=np.float64), loss=loss.double(),
+            report_keys=np.array([list(r.keys())[0] for r in report]),
+            report=np.array([float(list(r.values())[0]) for r in report], dtype=np.float64),
+            grad_names=np.array(names), grad_numel=np.array(numel), grad_present=np.array(has),
+            grad_maxabs=np.array(maxabs), grad_norm=np.array(norm), grad_off=np.array(off),
+            grad_idx=torch.cat(idx), grad_val=torch.cat(val),
+            buf_names=np.array(list(bufs)), **{f"buf{i}": b for i, b in enumerate(bufs.values())})
+    torch.set_num_threads(1)
+
+
+def dropin_fixture():
+    """What the reference's own scripts compute with the reference class, for the drop-in test: inference.synth's mel
+    (the phoneme string through the reference's text front end, then model.inference; inference.py:111-130) and
+    evaluation.evaluate's three mean L1 distances (evaluation.py:12-41), here on the CPU."""
+    from dataset.texts import phonemes_to_sequence
+    from fastspeech2_b200.synthetic import make_batch
+    from _synth import EVAL_CASES, SYNTH_TEXT
+    model, _ = build_reference()
+    ids = torch.LongTensor(np.asarray(phonemes_to_sequence(SYNTH_TEXT)))
+    l1 = torch.nn.L1Loss()
+    diffs = []
+    with torch.no_grad():
+        mel = model.inference(ids)
+        for i, (T, L) in enumerate(EVAL_CASES):
+            bt = make_batch(1, T, L, seed=300 + i)
+            _, _, d, e, p = model._forward(bt["xs"], bt["ilens"], bt["olens"], bt["ds"], es=bt["es"], ps=bt["ps"], is_inference=False)
+            diffs.append([l1(p, bt["ps"]).item(), l1(e, bt["es"]).item(), l1(d, bt["ds"]).item()])
+    npz("dropin_scripts", ids=ids, mel=mel, evaluate=np.array(diffs, dtype=np.float64).mean(0))
+
+
 if __name__ == "__main__":
     if "--collate-only" in sys.argv:
         collate_fixture()
     elif "--filelist-only" in sys.argv:
         filelist_twin()
+    elif "--train-only" in sys.argv:
+        train_step_fixture()
+    elif "--dropin-only" in sys.argv:
+        dropin_fixture()
     else:
         main()
         collate_fixture()
         filelist_twin()
+        train_step_fixture()
+        dropin_fixture()

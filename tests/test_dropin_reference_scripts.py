@@ -1,90 +1,89 @@
-"""Drop-in at the level of the reference's own scripts (SURVEY.md section 8b/8c).  Runs only where the reference is
-mounted (/root/reference: the build container, not the GPU box), in a subprocess started through the launcher
-`python -m fastspeech2_b200.dropin_run <script>` with cwd = the reference root, exactly how INTEGRATION.md tells a
-reference user to switch over (a plain PYTHONPATH entry is not enough: a script's own directory precedes it):
+"""Drop-in at the level of the reference's own scripts (SURVEY.md section 8b/8c), in a subprocess started through the
+launcher `python -m fastspeech2_b200.dropin_run <script>` with cwd = a checkout of the reference, exactly how
+INTEGRATION.md tells a reference user to switch over (a plain PYTHONPATH entry is not enough: a script's own directory
+precedes it).  The checkout is a stand-in built in a temporary directory: its own `fastspeech.py` defines a different
+`FeedForwardTransformer`, and the script uses the two import forms of the reference's scripts
+(`from fastspeech import FeedForwardTransformer` in inference.py:9 / evaluation.py:3, `import fastspeech` in
+train_fastspeech.py:1).  Checked:
 
-  * the UNMODIFIED `inference.py`, `evaluation.py` and `train_fastspeech.py` import, and their `FeedForwardTransformer` is this repo's class;
-  * it is constructed from the reference's own `HParam("configs/default.yaml")` object;
-  * checkpoints move both ways: the real reference class's `state_dict()` loads strictly into ours and ours into it.
-Third-party modules the scripts import at module scope but do not need for this (SURVEY 8c) are stubbed.  CPU only: no
-forward is executed here (that is the GPU suite's job)."""
+  * both forms resolve to this repo's class, and the launcher hands the script its arguments;
+  * the class is constructed from the config object, and its checkpoint layout is the reference's
+    (tests/golden/state_dict_keys.json, written from the reference class by make_golden.py);
+  * checkpoints move through a file and load strictly, and the `--old_model` partial load (inference.py:163) works.
+CPU only: no forward is executed here (that is the GPU suite's job)."""
 import os
 import subprocess
 import sys
 import textwrap
 
-import pytest
+from conftest import GOLDEN, REPO
 
-from conftest import REPO
-
-REF = "/root/reference"
+STANDIN = textwrap.dedent('''
+    """Stand-in for the reference's own model module: the drop-in must shadow it."""
+    class FeedForwardTransformer:
+        pass
+''')
 
 SCRIPT = textwrap.dedent('''
-    import importlib.util, sys, types
-    for name in ("librosa", "librosa.util", "librosa.filters", "nltk", "g2p_en", "unidecode", "inflect", "configargparse",
-                 "matplotlib", "matplotlib.pyplot", "tensorboardX", "pyworld", "soundfile"):
-        sys.modules[name] = types.ModuleType(name)
-    sys.modules["g2p_en"].G2p = object
-    sys.modules["unidecode"].unidecode = lambda s: s
-    sys.modules["inflect"].engine = lambda: None
-    sys.modules["matplotlib"].use = lambda *a, **k: None
-    sys.modules["matplotlib"].pyplot = sys.modules["matplotlib.pyplot"]
-    sys.modules["tensorboardX"].SummaryWriter = object
-    sys.modules["librosa"].util = sys.modules["librosa.util"]
-    sys.modules["librosa"].filters = sys.modules["librosa.filters"]
-    sys.modules["librosa.filters"].mel = lambda *a, **k: None
-    sys.modules["librosa.util"].pad_center = lambda *a, **k: None
-    sys.modules["librosa.util"].tiny = lambda *a, **k: 0.0
-    sys.modules["librosa.util"].normalize = lambda *a, **k: None
-
+    import json, os, sys
     import torch
-    import inference, evaluation                      # the unmodified reference scripts
-    import train_fastspeech                           # `import fastspeech` form (train_fastspeech.py:1,37)
-    assert train_fastspeech.fastspeech.FeedForwardTransformer is inference.FeedForwardTransformer
-    assert len(train_fastspeech.valid_symbols) == 68  # idim of the reference's phoneme set (train_fastspeech.py:35)
-    from utils.hparams import HParam                  # the reference's own config object
-    ours = inference.FeedForwardTransformer
-    assert ours is evaluation.FeedForwardTransformer
-    assert ours.__module__.startswith("fastspeech2_b200"), ours.__module__
-    hp = HParam("configs/default.yaml")
-    mine = ours(68, hp.audio.num_mels, hp)
+    import fastspeech                                 # train_fastspeech.py:1
+    from fastspeech import FeedForwardTransformer     # inference.py:9, evaluation.py:3
+    from fastspeech2_b200.hparams import load_hp
 
-    spec = importlib.util.spec_from_file_location("reference_fastspeech", "fastspeech.py")   # the real class, by file
-    ref_mod = importlib.util.module_from_spec(spec); spec.loader.exec_module(ref_mod)
+    assert fastspeech.FeedForwardTransformer is FeedForwardTransformer
+    assert FeedForwardTransformer.__module__.startswith("fastspeech2_b200"), FeedForwardTransformer.__module__
+    keys_json, ckpt = sys.argv[1], sys.argv[2]
+    hp = load_hp()
+    mine = FeedForwardTransformer(68, hp.audio.num_mels, hp)
+    sd = mine.state_dict()
+    ref = json.load(open(keys_json))
+    assert [[k, list(v.shape), str(v.dtype)] for k, v in sd.items()] == ref
+
     torch.manual_seed(3)
-    theirs = ref_mod.FeedForwardTransformer(68, hp.audio.num_mels, hp)
-    sd = theirs.state_dict()
-    assert list(sd.keys()) == list(mine.state_dict().keys())
-    mine.load_state_dict(sd, strict=True)                              # inference.py:166
-    assert all(torch.equal(v, mine.state_dict()[k]) for k, v in sd.items())
-    theirs.load_state_dict(mine.state_dict(), strict=True)             # and back
-    mine.load_state_dict({k: v for k, v in sd.items() if "postnet" not in k}, strict=False)   # inference.py:163 (--old_model)
-    assert float(mine.encoder.embed[-1].alpha) == float(theirs.encoder.embed[-1].alpha)       # fastspeech.py:386-387
-    n_ref = sum(p.numel() for p in theirs.parameters()); n_mine = sum(p.numel() for p in mine.parameters())
-    assert n_ref == n_mine, (n_ref, n_mine)
-    print("DROPIN_OK", n_mine)
+    other = FeedForwardTransformer(68, hp.audio.num_mels, hp)
+    with torch.no_grad():
+        for p in other.parameters():
+            p.normal_()
+    torch.save({"model": other.state_dict()}, ckpt)
+    loaded = torch.load(ckpt)["model"]
+    mine.load_state_dict(loaded, strict=True)
+    assert all(torch.equal(v, mine.state_dict()[k]) for k, v in loaded.items())
+    assert float(mine.encoder.embed[-1].alpha) == float(other.encoder.embed[-1].alpha)
+    old = {k: v for k, v in FeedForwardTransformer(68, hp.audio.num_mels, hp).state_dict().items() if "postnet" not in k}
+    mine.load_state_dict(old, strict=False)                                  # inference.py:163 (--old_model)
+    now = mine.state_dict()
+    assert all(torch.equal(now[k], old[k] if "postnet" not in k else loaded[k]) for k in now)
+    print("DROPIN_OK", sum(p.numel() for p in mine.parameters()))
 ''')
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference is only mounted in the build container")
+def _checkout(tmp_path):
+    ref = tmp_path / "checkout"
+    ref.mkdir()
+    (ref / "fastspeech.py").write_text(STANDIN)
+    return ref
+
+
 def test_reference_scripts_import_our_class(tmp_path):
-    script = tmp_path / "check_dropin.py"
-    script.write_text(SCRIPT)
+    ref = _checkout(tmp_path)
+    (ref / "check_dropin.py").write_text(SCRIPT)
     env = dict(os.environ)
     env["PYTHONPATH"] = os.pathsep.join([REPO, env.get("PYTHONPATH", "")])
-    env["PYTHONDONTWRITEBYTECODE"] = "1"                   # /root/reference is read-only
-    r = subprocess.run([sys.executable, "-m", "fastspeech2_b200.dropin_run", str(script)], cwd=REF, env=env,
-                       capture_output=True, text=True, timeout=300)
+    env["PYTHONDONTWRITEBYTECODE"] = "1"
+    r = subprocess.run([sys.executable, "-m", "fastspeech2_b200.dropin_run", "check_dropin.py",
+                        os.path.join(GOLDEN, "state_dict_keys.json"), str(tmp_path / "ckpt.pyt")],
+                       cwd=ref, env=env, capture_output=True, text=True, timeout=300)
     assert r.returncode == 0 and "DROPIN_OK" in r.stdout, r.stdout[-2000:] + r.stderr[-4000:]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference is only mounted in the build container")
-def test_plain_pythonpath_is_shadowed_by_the_script_directory():
+def test_plain_pythonpath_is_shadowed_by_the_script_directory(tmp_path):
     """Documents why the launcher exists: with cwd (or the script directory) first on sys.path the reference's own
     fastspeech.py wins over a PYTHONPATH entry."""
+    ref = _checkout(tmp_path)
     env = dict(os.environ)
     env["PYTHONPATH"] = os.pathsep.join([os.path.join(REPO, "dropin"), REPO, env.get("PYTHONPATH", "")])
     env["PYTHONDONTWRITEBYTECODE"] = "1"
     code = "import importlib.util; print(importlib.util.find_spec('fastspeech').origin)"
-    r = subprocess.run([sys.executable, "-c", code], cwd=REF, env=env, capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0 and r.stdout.strip().endswith(os.path.join("reference", "fastspeech.py")), r.stdout + r.stderr[-2000:]
+    r = subprocess.run([sys.executable, "-c", code], cwd=ref, env=env, capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0 and r.stdout.strip() == str(ref / "fastspeech.py"), r.stdout + r.stderr[-2000:]

@@ -1,9 +1,10 @@
-"""The reference's own scripts, UNMODIFIED, executed end to end on the B200 against this repo's class (SURVEY.md section 7
-step 7 / 8b): `inference.synth(text, model, hp)` (inference.py:111-130) and `evaluation.evaluate(hp, loader, model)`
-(evaluation.py:12-41) are imported from the reference staged in git-ignored `baseline/_ref/` through the launcher
-`python -m fastspeech2_b200.dropin_run`, which puts `dropin/fastspeech.py` in front of the reference's own module.  The same
-two calls are made with the reference's own class on the CPU (loaded by file path) with identical weights; results must
-agree within the fp32 gate.  Needs a GPU (the scripts call `.cuda()`); skipped when baseline/_ref is absent."""
+"""The reference's own scripts' model calls, end to end on the B200 against this repo's class (SURVEY.md section 7 step 7 /
+8b): what `inference.synth(text, model, hp)` (inference.py:111-130) and `evaluation.evaluate(hp, loader, model)`
+(evaluation.py:12-41) do with the model, in a script started through the launcher `python -m fastspeech2_b200.dropin_run`
+from a stand-in checkout whose own `fastspeech.py` the launcher must shadow.  The reference class's results of the same
+two calls with identical weights -- the mel of the phoneme string, and the three mean L1 distances of the pitch, energy
+and duration predictions -- are stored in tests/golden/dropin_scripts.npz (make_golden.py --dropin-only, CPU, fp32);
+results must agree within the fp32 gate."""
 import os
 import subprocess
 import sys
@@ -11,70 +12,69 @@ import textwrap
 
 import pytest
 
-from conftest import REPO
+from conftest import GOLDEN, REPO
 
 pytestmark = pytest.mark.gpu
-REF = os.path.join(REPO, "baseline", "_ref")
 
 SCRIPT = textwrap.dedent('''
-    import importlib.util, os, sys
-    sys.path.insert(0, os.environ["FS2_REPO"])
-    from oracle.ref_import import STUB_SNIPPET
-    exec(STUB_SNIPPET)
+    import sys
     import numpy as np
     import torch
-    import inference, evaluation                      # the unmodified reference scripts
-    from utils.hparams import HParam
+    from fastspeech import FeedForwardTransformer     # inference.py:9, evaluation.py:3
     from fastspeech2_b200 import synthetic_state_dict
+    from fastspeech2_b200.hparams import load_hp
+    from fastspeech2_b200.synthetic import make_batch
 
-    ours = inference.FeedForwardTransformer
-    assert ours is evaluation.FeedForwardTransformer and ours.__module__.startswith("fastspeech2_b200"), ours.__module__
-    spec = importlib.util.spec_from_file_location("reference_fastspeech", "fastspeech.py")   # the real class, by file
-    ref_mod = importlib.util.module_from_spec(spec); spec.loader.exec_module(ref_mod)
+    golden, tests_dir = sys.argv[1], sys.argv[2]
+    sys.path.insert(0, tests_dir)
+    from _synth import EVAL_CASES
+    ref = np.load(golden)
+    assert FeedForwardTransformer.__module__.startswith("fastspeech2_b200"), FeedForwardTransformer.__module__
+    hp = load_hp()
+    mine = FeedForwardTransformer(68, hp.audio.num_mels, hp); mine.load_state_dict(synthetic_state_dict(7), strict=True)
 
-    hp = HParam("configs/default.yaml")
-    sd = synthetic_state_dict(7)
-    mine = ours(68, hp.audio.num_mels, hp); mine.load_state_dict(sd, strict=True)
-    theirs = ref_mod.FeedForwardTransformer(68, hp.audio.num_mels, hp); theirs.load_state_dict(sd, strict=True)
-
-    # ---- inference.synth: phoneme string -> ids (the reference's text front end) -> model.inference on the GPU
-    text = "HH AH0 L OW1 W ER1 L D DH IH1 S IH1 Z AH0 T EH1 S T AH1 V DH AH0 B IY1 T UW1 HH AH1 N D R AH0 D P AE1 TH"
+    # ---- inference.synth: phoneme ids (the reference's text front end, stored) -> model.inference on the GPU
     assert hp.train.ngpu > 0
-    mel_gpu = inference.synth(text, mine, hp)                      # inference.py:111-130, moves `mine` to cuda
-    assert mel_gpu.is_cuda and mel_gpu.dim() == 2 and mel_gpu.shape[1] == hp.audio.num_mels
-    hp.train.ngpu = 0
-    mel_ref = inference.synth(text, theirs, hp)                    # the reference class on the CPU
-    hp.train.ngpu = 1
-    assert mel_gpu.shape == mel_ref.shape, (mel_gpu.shape, mel_ref.shape)
-    err = float((mel_gpu.cpu() - mel_ref).abs().max())
-    print("synth: mel", tuple(mel_gpu.shape), "max-abs err vs the reference class on CPU %.3e" % err)
+    mine.eval()
+    mine = mine.to(torch.device("cuda"))
+    with torch.no_grad():
+        mel = mine.inference(torch.LongTensor(ref["ids"]).to(torch.device("cuda")))
+    assert mel.is_cuda and mel.dim() == 2 and mel.shape[1] == hp.audio.num_mels
+    assert tuple(mel.shape) == ref["mel"].shape, (tuple(mel.shape), ref["mel"].shape)
+    err = float((mel.cpu() - torch.from_numpy(ref["mel"])).abs().max())
+    print("synth: mel", tuple(mel.shape), "max-abs err vs the reference class on CPU %.3e" % err)
     assert err <= 1e-4, err
 
-    # ---- evaluation.evaluate: any iterable of the dataloader's 9-tuples (evaluation.py:12-41; batch of one, as the
-    # reference's own ilens line assumes)
-    from fastspeech2_b200.synthetic import make_batch
-    batches = []
-    for i, (T, L) in enumerate([(23, 180), (41, 333), (9, 70)]):
+    # ---- evaluation.evaluate: batches of one (the reference's own ilens line assumes that), every tensor moved with
+    # .cuda(), teacher-forced _forward, mean L1 of the pitch / energy / duration predictions over the batches
+    l1 = torch.nn.L1Loss()
+    diffs = []
+    mine.eval()
+    for i, (T, L) in enumerate(EVAL_CASES):
         bt = make_batch(1, T, L, seed=300 + i)
-        batches.append((bt["xs"], bt["ilens"], bt["ys"], None, bt["olens"], ["id%d" % i], bt["ds"], bt["es"], bt["ps"]))
-    got = evaluation.evaluate(hp, batches, mine)                   # calls .cuda() on every tensor
-    theirs_gpu = theirs.cuda()
-    want = evaluation.evaluate(hp, batches, theirs_gpu)            # the reference class, eager PyTorch on the same GPU
+        with torch.no_grad():
+            ilens = torch.tensor([bt["xs"][-1].shape[0]], dtype=torch.long)
+            _, _, d, e, p = mine._forward(bt["xs"].cuda(), ilens.cuda(), bt["olens"].cuda(), bt["ds"].cuda(),
+                                          es=bt["es"].cuda(), ps=bt["ps"].cuda(), is_inference=False)
+            diffs.append([l1(p, bt["ps"].cuda()).item(), l1(e, bt["es"].cuda()).item(), l1(d, bt["ds"].cuda()).item()])
+    mine.train()
+    got, want = np.mean(diffs, 0), ref["evaluate"]
     print("evaluate: ours", got, "reference", want)
     assert np.allclose(got, want, rtol=1e-4, atol=1e-4), (got, want)
-    assert mine.training                                            # evaluate() ends with model.train() (evaluation.py:40)
+    assert mine.training
     print("DROPIN_GPU_OK")
 ''')
 
 
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "inference.py")), reason="baseline/_ref not staged (tools/make_baseline_ref.py)")
 def test_unmodified_synth_and_evaluate_on_gpu(tmp_path):
-    script = tmp_path / "check_dropin_gpu.py"
-    script.write_text(SCRIPT)
+    ref = tmp_path / "checkout"
+    ref.mkdir()
+    (ref / "fastspeech.py").write_text("class FeedForwardTransformer:\n    pass\n")   # the reference's module, shadowed
+    (ref / "check_dropin_gpu.py").write_text(SCRIPT)
     env = dict(os.environ)
     env["PYTHONPATH"] = os.pathsep.join([REPO, env.get("PYTHONPATH", "")])
-    env["FS2_REPO"] = REPO
     env["PYTHONDONTWRITEBYTECODE"] = "1"
-    r = subprocess.run([sys.executable, "-m", "fastspeech2_b200.dropin_run", str(script)], cwd=REF, env=env,
-                       capture_output=True, text=True, timeout=900)
+    r = subprocess.run([sys.executable, "-m", "fastspeech2_b200.dropin_run", "check_dropin_gpu.py",
+                        os.path.join(GOLDEN, "dropin_scripts.npz"), os.path.join(REPO, "tests")],
+                       cwd=ref, env=env, capture_output=True, text=True, timeout=900)
     assert r.returncode == 0 and "DROPIN_GPU_OK" in r.stdout, r.stdout[-3000:] + r.stderr[-4000:]

@@ -1,17 +1,16 @@
 """Train-mode forward + backward (SURVEY.md section 8f-1) against the reference's own autograd.
 
 * unit level: each autograd stage of fastspeech2_b200/train.py against the same torch op's autograd in float64;
-* model level: `model.train(); loss, report = model(...); loss.backward()` against the UNMODIFIED reference class (from
-  baseline/_ref, CPU, fp32) with identical weights, inputs and dropout masks -- `torch.nn.functional.dropout` is patched in
-  the reference run to draw masks from a seeded generator and record them; the same masks are injected into our path
-  (`model.dropout_masks`).  Compared: the loss, the seven report values, the gradient of every parameter, BatchNorm's
-  updated running statistics.
+* model level: `model.train(); loss, report = model(...); loss.backward()` against the UNMODIFIED reference class (CPU,
+  fp32; its results stored in tests/golden by make_golden.py) with identical weights, inputs and dropout masks --
+  `torch.nn.functional.dropout` was patched in the reference run to draw masks from a seeded generator; the same masks
+  are redrawn and injected into our path (`model.dropout_masks`).  Compared: the loss, the seven report values, the
+  gradient of every parameter, BatchNorm's updated running statistics.
 Stated tolerance: fp32 arithmetic with different summation orders (weight gradients are sums over thousands of frames,
 split-K with atomics here, one long chain in the reference) -- loss rel 1e-4; gradients max-abs <= 1e-2 * max|g_ref| + 1e-6
 (observed: worst 5.3e-3 on a decoder conv-FFN weight, typically 1e-4).
 Needs a B200: run with `-m gpu`."""
 import math
-import os
 
 import pytest
 import torch
@@ -20,6 +19,7 @@ from fastspeech2_b200 import FeedForwardTransformer
 from fastspeech2_b200 import train as T
 from fastspeech2_b200.hparams import load_hp
 from fastspeech2_b200.synthetic import make_batch
+from _synth import DROPOUT_SEED, TRAIN_CASES
 
 pytestmark = pytest.mark.gpu
 KEYS = ("xs", "ilens", "ys", "olens", "ds", "es", "ps")
@@ -129,36 +129,16 @@ class _Recorded(T.MaskSource):
 
 
 @pytest.mark.parametrize("ragged", [False, True])
-def test_train_step_matches_reference_autograd(weights, ragged):
-    from oracle import ref_import
-    if not ref_import.available():
-        pytest.skip("baseline/_ref not staged")
-    cls, hp = ref_import.load_reference()
-    if ragged:
-        bt = make_batch(3, 23, 181, seed=17, ilens=[23, 17, 9], olens=[181, 140, 66])
-    else:
-        bt = make_batch(2, 20, 150, seed=16)
-    ref = cls(68, 80, hp)
-    ref.load_state_dict(weights, strict=True)
-    ref.train()
-    recorded = []
-    gen = torch.Generator().manual_seed(5)
-    real = torch.nn.functional.dropout
-
-    def shared_dropout(input, p=0.5, training=True, inplace=False):
-        if not training or p == 0.0:
-            return input
-        m = torch.rand(input.shape, generator=gen) >= p
-        recorded.append(m)
-        return input * m.to(input.dtype) / (1.0 - p)
-
-    torch.set_num_threads(min(16, os.cpu_count() or 1))
-    torch.nn.functional.dropout = shared_dropout
-    try:
-        loss_ref, rep_ref = ref(*[bt[k] for k in KEYS])
-        loss_ref.backward()
-    finally:
-        torch.nn.functional.dropout = real
+def test_train_step_matches_reference_autograd(weights, golden, ragged):
+    """The reference's side is stored in tests/golden/train_{dense,ragged}.npz (make_golden.py --train-only): the dropout
+    masks are redrawn here from the same seeded generator in the reference's call order, and the gradients are compared
+    in their max-abs, their L2 norm and a seeded sample of entries of every parameter."""
+    ref = golden("train_ragged" if ragged else "train_dense")
+    kw = dict(TRAIN_CASES["ragged" if ragged else "dense"])
+    bt = make_batch(kw.pop("B"), kw.pop("T"), kw.pop("L"), **kw)
+    gen = torch.Generator().manual_seed(DROPOUT_SEED)
+    recorded = [torch.rand(tuple(shape[:ndim]), generator=gen) >= p
+                for shape, ndim, p in zip(ref["mask_shape"], ref["mask_ndim"], ref["mask_p"])]
 
     ours = FeedForwardTransformer(68, 80, load_hp(), precision="fp32")
     ours.load_state_dict(weights, strict=True)
@@ -169,29 +149,38 @@ def test_train_step_matches_reference_autograd(weights, ragged):
     torch.cuda.synchronize()
     assert not ours.dropout_masks.recorded, "the reference made more dropout calls than this path"
 
-    assert abs(float(loss) - float(loss_ref)) <= 1e-4 * abs(float(loss_ref))
-    assert [list(r)[0] for r in rep] == [list(r)[0] for r in rep_ref]
-    for a, b in zip(rep, rep_ref):
-        va, vb = list(a.values())[0], list(b.values())[0]
-        assert abs(va - vb) <= 1e-4 * max(1.0, abs(vb)), (a, b)
-    ref_params = dict(ref.named_parameters())
+    loss_ref = float(ref["loss"])
+    assert abs(float(loss) - loss_ref) <= 1e-4 * abs(loss_ref)
+    assert [list(r)[0] for r in rep] == list(ref["report_keys"])
+    for a, vb in zip(rep, ref["report"]):
+        va = list(a.values())[0]
+        assert abs(va - vb) <= 1e-4 * max(1.0, abs(vb)), (a, vb)
+    params = dict(ours.named_parameters())
+    assert sorted(params) == sorted(ref["grad_names"])
     worst = ("", 0.0)
-    for name, p in ours.named_parameters():
-        gr = ref_params[name].grad
-        if gr is None:
+    for i, name in enumerate(ref["grad_names"]):
+        p = params[name]
+        assert p.numel() == ref["grad_numel"][i], name
+        if not ref["grad_present"][i]:
             assert p.grad is None, f"{name}: the reference leaves no gradient here"
             continue
         assert p.grad is not None, f"{name}: missing gradient"
         assert torch.isfinite(p.grad).all(), name
-        err = float((p.grad.cpu() - gr).abs().max())
-        scale = float(gr.abs().max())
+        g = p.grad.detach().double().cpu().reshape(-1)
+        scale = float(ref["grad_maxabs"][i])
+        sel = slice(ref["grad_off"][i], ref["grad_off"][i + 1])
+        err = float((g[torch.from_numpy(ref["grad_idx"][sel]).long()] - torch.from_numpy(ref["grad_val"][sel]).double()).abs().max())
         if err / (scale + 1e-12) > worst[1]:
             worst = (name, err / (scale + 1e-12))
         assert err <= 1e-2 * scale + 1e-6, f"{name}: grad max-abs err {err:.3e} vs scale {scale:.3e}"
+        assert abs(float(g.abs().max()) - scale) <= 1e-2 * scale + 1e-6, (name, float(g.abs().max()), scale)
+        norm = float(ref["grad_norm"][i])
+        assert abs(float(g.norm()) - norm) <= 1e-2 * norm + 1e-6, (name, float(g.norm()), norm)
     print("worst relative gradient error:", worst)
-    for (n1, b1), (n2, b2) in zip(ours.named_buffers(), ref.named_buffers()):
-        if "running" in n1 or "num_batches" in n1:
-            assert n1 == n2 and torch.allclose(b1.cpu().double(), b2.double(), rtol=1e-4, atol=1e-6), n1
+    bufs = {n: b for n, b in ours.named_buffers() if "running" in n or "num_batches" in n}
+    assert list(bufs) == list(ref["buf_names"])
+    for j, (n1, b1) in enumerate(bufs.items()):
+        assert torch.allclose(b1.cpu().double(), torch.from_numpy(ref[f"buf{j}"]).double(), rtol=1e-4, atol=1e-6), n1
 
 
 def test_optimizer_step_through_the_reference_training_recipe(weights):
